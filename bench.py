@@ -1,6 +1,6 @@
 """bench.py — SCAIL-14B denoising steps/sec at 512p/81f (config A of BASELINE.json / SURVEY §8d).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one sampler step of the reference (sgm/modules/diffusionmodules/sampling.py:950-963): the
 CFG-duplicated batch-2 DiT forward over the ref || noise || pose sequence (N = 27 904 tokens, 40 blocks,
@@ -24,8 +24,13 @@ by the 40 layers x 2 CFG branches it stands for (machine-readable: cpu_baseline.
 actually runs on a GPU (cuBLASLt F.linear, flash/cuDNN SDPA, F.layer_norm; baseline/torchlib.py).  The default arm
 also times it after its own timed region and reports `library_baseline`, plus per-kernel `kernel_compare`
 (ours vs cuBLAS / SDPA at the step's shapes) and `vae_decode` (config 5, ours vs cuDNN conv3d) at N=1.
+
+--dump-outputs DIR (GPU arms): after the timed steps, rank 0 writes the fp32 latent the last timed step returned as
+DIR/latent.npy.  Weights and inputs are seeded, so two builds run with the same arguments can be compared output for
+output.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -36,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: importing the package must not write __pycache__ into it
 
 import torch  # noqa: E402
 
@@ -79,6 +85,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.QUERY}", "--format=csv,noheader,nounits",
                                           "-lms", "200", "-i", str(self.index)], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.terminate)  # the poller never ends by itself: stop it even if the run raises
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -91,6 +98,11 @@ class ClockSampler:
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        try:
+            self.proc.wait(timeout=5)
+        except subprocess.TimeoutExpired:
+            self.proc.kill()
+            self.proc.wait()
         time.sleep(0.05)
         sm, mx, reasons = [], [], set()
         for r in self.rows:
@@ -333,6 +345,23 @@ def cp_consistency_check(model, d, cond, uc, sig, rank, dist, plan=None, layers=
     return rel
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy in float32, all of them together within DUMP_MAX_BYTES.  A tensor over its
+    share is replaced by a fixed seeded sample of its flattened elements (the same positions on every run of one shape)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_MAX_BYTES // len(arrays) // 4
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > share:
+            idx = torch.randint(a.numel(), (share,), generator=torch.Generator().manual_seed(0)).sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
 def parallelism_name(n_gpus, mode="auto"):
     if n_gpus <= 1:
         return "single"
@@ -365,7 +394,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--latent", default=None, help="TxHxW latent override, e.g. 21x64x112 (the reference's default 512x896); "
                     "the default 21x64x64 is the BASELINE.json config")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the latent the last timed step "
+                    "returned as DIR/latent.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arms (--impl ours|torchlib)")
     if args.latent:
         global T_LAT, H_LAT, W_LAT
         T_LAT, H_LAT, W_LAT = (int(v) for v in args.latent.lower().split("x"))
@@ -451,7 +486,7 @@ def main():
         t0 = torch.cuda.Event(enable_timing=True); t1 = torch.cuda.Event(enable_timing=True)
         t0.record()
         for i in range(args.steps):
-            hs(sig[i], sig[i + 1])
+            hs(sig[i % 50], sig[i % 50 + 1])
         t1.record()
         barrier()
         e2e_ms = t0.elapsed_time(t1) / args.steps
@@ -492,6 +527,8 @@ def main():
                         "algorithmic_flops_per_launch": attn_flops, "avg_launch_ms": attn_avg,
                         "share_of_step": sum(attn_ms) / args.steps / ms if attn_ms else None}}
     out["latent_checksum"] = float(x.double().abs().mean())  # same seeded inputs => comparable across N and across arms
+    if args.dump_outputs:  # x still holds the last timed step's output: the e2e run above used its own buffers
+        dump_outputs(args.dump_outputs, {"latent": x})
     if cp_check is not None:
         out["cp_check_rel"] = cp_check
     if args.layers != LAYERS:

@@ -14,6 +14,8 @@ Outputs (committed, small):
   tests/golden/sampler.pt      — sigma schedule make_flow_timesteps(0,50,shift 5), CFG+Euler step.
   tests/golden/vae_small.pt    — WanVAE_ decode of a [1,16,3,8,8] latent (dim=16 narrow variant
                                  of the same architecture), state_dict + output.
+  tests/golden/mixin_surface.json — the reference's DiffusionTransformer built with its mixin targets
+                                 pointed at scail_b200.dit: mixin classes, hook origins, parameter shapes.
 The GPU box never runs this (no /root/reference there); tests read the .pt files.
 """
 import os
@@ -152,9 +154,35 @@ def gen_vae():
     return res
 
 
+def gen_mixin_surface():
+    """What the reference's own DiffusionTransformer makes of scail_b200.dit when the YAML `target:` strings point at it:
+    the module and class of every mixin it instantiated, the mixin each SAT hook was collected from
+    (BaseModel.collect_hooks_), and the stock model's parameter shapes (which the plugged-in model must reproduce)."""
+    import importlib
+    import json
+    H.setup()
+    import dit_video_crossattn_sc_xc as ref
+    import scail_b200.dit as ours
+    importlib.reload(ours)  # real SAT BaseMixins now that SAT is importable
+    cfg = dict(hidden=256, heads=2, inner=512, layers=1, text_dim=64)
+    stock = ref.DiffusionTransformer(**H.dit_config(**cfg))
+    mine = ref.DiffusionTransformer(**H.dit_config(mixin_module="scail_b200.dit", **cfg))
+    shapes = {k: list(v.shape) for k, v in stock.state_dict().items()}
+    assert {k: list(v.shape) for k, v in mine.state_dict().items()} == shapes
+    surface = {"config": cfg, "param_shapes": shapes,
+               "mixins": {k: [type(m).__module__, type(m).__name__] for k, m in mine.mixins.items()},
+               "hook_origins": dict(mine.hook_origins)}
+    with open(os.path.join(OUT, "mixin_surface.json"), "w") as f:
+        json.dump(surface, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("mixin surface:", surface["hook_origins"])
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["dit", "vae"]
+    which = sys.argv[1:] or ["dit", "vae", "mixins"]
     if "dit" in which:
         gen_dit()
     if "vae" in which:
         gen_vae()
+    if "mixins" in which:
+        gen_mixin_surface()
